@@ -210,6 +210,28 @@ def run_reference(args):
 # ------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(dirpath: str, fitted) -> None:
+    """Writes the fitted-model arrays of the last timed step (host FittedBatch) as DIR/<field>.npy in float64, so that
+    two builds can be compared output for output.  The integers are exact in float64: int32 always, and the int64
+    start / scale timestamps because the synthetic grid is whole 15-min steps from midnight (multiples of 2**11 ns).
+    Above DUMP_LIMIT_BYTES a fixed seeded sample of series (rows) is written, with its row indices in series_index.npy."""
+    arrays = {name: np.asarray(getattr(fitted, name)).astype(np.float64)
+              for name in ("params", "tchange", "meta_i32", "meta_i64", "meta_f64")}
+    n = fitted.n
+    row_bytes = 8 * sum(a.shape[1] for a in arrays.values())
+    budget = DUMP_LIMIT_BYTES - 4096                    # room for the .npy headers
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["series_index"] = rows.astype(np.float64)
+    os.makedirs(dirpath, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirpath, f"{name}.npy"), a)
+
+
 def _kernel_name(variants: dict, group_g: int, opts_growth_logistic=True) -> str:
     """The dominant fit kernel of the last step from the variant counts the library reports."""
     if not variants:
@@ -413,6 +435,8 @@ def run_gpu(args):
     if cpu is not None:
         line["cpu_baseline"] = cpu
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, host)
     if world > 1:
         dist.destroy_process_group()
     return 0
@@ -558,7 +582,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="what `value` means at N > 1: the same 50k series split over the ranks (north_star), or 50k per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the run, write the fitted-model arrays of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes one GPU's fit: use it with --impl b200 on a single rank")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

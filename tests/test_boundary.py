@@ -229,7 +229,9 @@ def test_big_forecast_frame_is_written_as_parallel_part_files(tmp_path, monkeypa
                     "dim_id": pa.array(np.repeat(np.arange(n_models, dtype=np.int32) % 5, H)),
                     "ds": pa.array(np.tile(grid, n_models)).cast(pa.timestamp("ns")),
                     "yhat": pa.array(rng.randint(0, 10**6, n_models * H).astype(np.int32))})
-    cfg = lambda d: {"io": {"models": "unused", "forecasts": str(tmp_path / d)}, "forecast": {"periods": H, "frequency": "15min"}}
+    # the Arrow writer's split: under the default writer (auto) a big frame goes to the GPU formatter where CUDA is present
+    cfg = lambda d: {"io": {"models": "unused", "forecasts": str(tmp_path / d)},
+                     "forecast": {"periods": H, "frequency": "15min", "writer": "arrow"}}
     frame = ProphetScorer.convert_forecasts(Frame(tbl))
     ProphetScorer(cfg("one")).write_forecasts(frame)
     monkeypatch.setattr(ps, "_ROWS_PER_PART", 300)

@@ -5,7 +5,7 @@ profiles/r2g_fit_group_g8_by_function.txt holds).  Usage (CPU box):
     nvdisasm -g -c fit_group_inst.sm_100a.cubin | awk '<keep the section of the captured kernel>' > /tmp/g8_lines.txt
     python tools/ncu_by_function.py
 (the kernel must have been compiled with -lineinfo; paths are the ones used above)."""
-import re, csv, sys, collections
+import re, csv, sys, collections, os
 # map offset -> (file, line, inline chain top function?) from nvdisasm -g output
 cur=None; off2line={}
 for ln in open('/tmp/g8_lines.txt'):
@@ -20,7 +20,7 @@ hdr=rows[1]; ia=hdr.index('Address'); isamp=hdr.index('# Samples'); iex=hdr.inde
 cols={k:hdr.index(k) for k in ['stall_wait','stall_no_inst','stall_short_sb','stall_long_sb','stall_branch_resolving','stall_selected','stall_not_selected','stall_math','stall_dispatch']}
 base=int(rows[2][ia],16)
 # function ranges in fit_group.cuh by line numbers
-src=open('/root/repo/time_series_spark_b200/csrc/fit_group.cuh').read().split('\n')
+src=open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'time_series_spark_b200', 'csrc', 'fit_group.cuh')).read().split('\n')
 funcs=[]
 for i,l in enumerate(src,1):
     m=re.match(r'(?:__device__|__global__|template).*?\b(g_\w+|gvdot|fit_group_kernel|day_features|gsum|gmax|gscan_excl\w*)\(', l)
