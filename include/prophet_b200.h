@@ -271,6 +271,39 @@ PB200_API int pb200_forecast_csv_rows_device(pb200_ctx* ctx, const int32_t* d_se
 PB200_API int32_t pb200_forecast_csv_row_host(int32_t series_id, int32_t dim_id, int64_t ds_ns, int32_t quantity,
                                               const char* created, int32_t created_len, char* out);
 
+/*
+ * The modeler's input CSV parsed on the device: header-less lines "dim_id,timestamp,quantity" (reference
+ * src/jobs/prophet_modeler.py:12-17,102-116) of files concatenated into one byte buffer d_text, every file ending in
+ * '\n'.  d_text is 16-byte aligned and readable up to n_bytes rounded up to 16 (the bytes past n_bytes are ignored).
+ * Accepted grammar, everything else is refused:
+ *     dim_id     -?[0-9]{1,10} within int32
+ *     timestamp  YYYY-MM-DD[ T]HH:MM:SS with an optional '.' and 1..9 fraction digits; year 1900..2199, a valid
+ *                calendar date, hour < 24, minute < 60, second < 60
+ *     quantity   -?[0-9]{1,10} within int32, or empty (null: quantity 0, valid 0)
+ *     line end   "\n" or "\r\n"
+ * Passes, in order on the context's stream:
+ *   count  d_tile_count[t] = newlines in bytes [t*PB200_INPUT_CSV_TILE, (t+1)*PB200_INPUT_CSV_TILE)
+ *          (ceil(n_bytes / PB200_INPUT_CSV_TILE) tiles);
+ *   index  given d_tile_off = exclusive scan of the tile counts, d_row_end[r] = offset one past row r's '\n'
+ *          (n_rows = sum of the tile counts);
+ *   parse  row r starts at d_row_end[r-1] (0 for r = 0); it belongs to the last file f with d_file_start[f] <= that
+ *          offset (d_file_start ascending) and gets series_id d_file_sid[f].  Writes the four columns and the
+ *          quantity valid mask; d_refused[0] = rows refused, d_refused[1] = index of the first refused row or -1.
+ *          A refused row's column values are unspecified.
+ * pb200_input_csv_row_host runs the same row parser on the host for ONE line of len bytes (its line end included):
+ * 1 accepted, 0 refused, -1 bad argument.
+ */
+#define PB200_INPUT_CSV_TILE 4096
+PB200_API int pb200_input_csv_count_device(pb200_ctx* ctx, const uint8_t* d_text, int64_t n_bytes, int64_t* d_tile_count);
+PB200_API int pb200_input_csv_index_device(pb200_ctx* ctx, const uint8_t* d_text, int64_t n_bytes,
+                                           const int64_t* d_tile_off, int64_t* d_row_end);
+PB200_API int pb200_input_csv_parse_device(pb200_ctx* ctx, const uint8_t* d_text, const int64_t* d_row_end, int64_t n_rows,
+                                           const int64_t* d_file_start, const int32_t* d_file_sid, int32_t n_files,
+                                           int32_t* d_series_id, int32_t* d_dim_id, int64_t* d_ds_ns, int32_t* d_quantity,
+                                           uint8_t* d_quantity_valid, int64_t* d_refused);
+PB200_API int32_t pb200_input_csv_row_host(const char* line, int64_t len, int32_t* dim_id, int64_t* ds_ns,
+                                           int32_t* quantity, int32_t* quantity_valid);
+
 #ifdef __cplusplus
 }
 #endif

@@ -49,7 +49,9 @@ EXPORTS = [
     "pb200_stream", "pb200_launch_count", "pb200_last_fit_variant_counts", "pb200_tab_chunk", "pb200_fit_device", "pb200_fit_host", "pb200_predict_device",
     "pb200_predict_host", "pb200_make_future_device", "pb200_synchronize", "pb200_objective_host",
     "pb200_fit_trace_host", "pb200_forecast_csv_lengths_device", "pb200_forecast_csv_rows_device", "pb200_forecast_csv_row_host",
+    "pb200_input_csv_count_device", "pb200_input_csv_index_device", "pb200_input_csv_parse_device", "pb200_input_csv_row_host",
 ]
+INPUT_CSV_TILE = 4096       # PB200_INPUT_CSV_TILE
 
 _lib = None
 
@@ -106,6 +108,14 @@ def load() -> C.CDLL:
     lib.pb200_forecast_csv_rows_device.restype = C.c_int
     lib.pb200_forecast_csv_row_host.argtypes = [i32, i32, i64, i32, C.c_char_p, i32, C.c_char_p]
     lib.pb200_forecast_csv_row_host.restype = i32
+    lib.pb200_input_csv_count_device.argtypes = [vp, vp, i64, vp]
+    lib.pb200_input_csv_count_device.restype = C.c_int
+    lib.pb200_input_csv_index_device.argtypes = [vp, vp, i64, vp, vp]
+    lib.pb200_input_csv_index_device.restype = C.c_int
+    lib.pb200_input_csv_parse_device.argtypes = [vp, vp, vp, i64, vp, vp, i32, vp, vp, vp, vp, vp, vp]
+    lib.pb200_input_csv_parse_device.restype = C.c_int
+    lib.pb200_input_csv_row_host.argtypes = [C.c_char_p, i64, vp, vp, vp, vp]
+    lib.pb200_input_csv_row_host.restype = i32
     lib.pb200_synchronize.argtypes = [vp]
     lib.pb200_synchronize.restype = C.c_int
     _lib = lib

@@ -248,6 +248,60 @@ def forecast_csv_row_host(series_id: int, dim_id: int, ds_ns: int, quantity: int
     return buf.raw[:n]
 
 
+def parse_input_csv_device(ctx: L.Context, text, n_bytes: int, file_start, file_sid):
+    """The modeler's input CSV parsed on the GPU (pb200_input_csv_{count,index,parse}_device): ``text`` a uint8 CUDA
+    tensor holding the concatenated files in its first ``n_bytes`` (every file ending in '\\n', numel a multiple of 16),
+    ``file_start`` / ``file_sid`` int64 / int32 CUDA tensors with each file's first byte and series_id.  Returns
+    (series_id, dim_id, ds_ns, quantity, quantity_valid, row_end, n_refused, first_refused): six CUDA tensors of one
+    entry per row (row_end: the offset one past the row's '\\n') and two ints (first_refused is -1 when no row was
+    refused).  Grammar: include/prophet_b200.h."""
+    import torch
+    dev = text.device
+    if text.dtype != torch.uint8 or not text.is_contiguous() or text.numel() % 16 or text.numel() < n_bytes:
+        raise ValueError("parse_input_csv_device wants a contiguous uint8 tensor padded to a multiple of 16 bytes")
+    lib = L.load()
+    tiles = -(-n_bytes // L.INPUT_CSV_TILE)
+    counts = torch.empty(tiles, dtype=torch.int64, device=dev)
+    torch.cuda.current_stream(dev).synchronize()
+    L.check(lib.pb200_input_csv_count_device(ctx.handle, text.data_ptr(), n_bytes, counts.data_ptr()),
+            "pb200_input_csv_count_device")
+    ctx.synchronize()
+    ends = torch.cumsum(counts, 0)                    # the scan is plumbing (torch); the passes over the bytes are the kernels
+    n_rows = int(ends[-1].item()) if tiles else 0
+    row_end = torch.empty(n_rows, dtype=torch.int64, device=dev)
+    offs = ends - counts
+    torch.cuda.current_stream(dev).synchronize()
+    L.check(lib.pb200_input_csv_index_device(ctx.handle, text.data_ptr(), n_bytes, offs.data_ptr(), row_end.data_ptr()),
+            "pb200_input_csv_index_device")
+    del counts, ends, offs
+    sid = torch.empty(n_rows, dtype=torch.int32, device=dev)
+    did = torch.empty(n_rows, dtype=torch.int32, device=dev)
+    ds = torch.empty(n_rows, dtype=torch.int64, device=dev)
+    qty = torch.empty(n_rows, dtype=torch.int32, device=dev)
+    valid = torch.empty(n_rows, dtype=torch.uint8, device=dev)
+    refused = torch.empty(2, dtype=torch.int64, device=dev)
+    torch.cuda.current_stream(dev).synchronize()
+    L.check(lib.pb200_input_csv_parse_device(ctx.handle, text.data_ptr(), row_end.data_ptr(), n_rows, file_start.data_ptr(),
+                                             file_sid.data_ptr(), int(file_start.numel()), sid.data_ptr(), did.data_ptr(),
+                                             ds.data_ptr(), qty.data_ptr(), valid.data_ptr(), refused.data_ptr()),
+            "pb200_input_csv_parse_device")
+    ctx.synchronize()
+    n_bad, first = (int(v) for v in refused.cpu().tolist())
+    return sid, did, ds, qty, valid, row_end, n_bad, first
+
+
+def input_csv_row_host(line: bytes):
+    """One input line, its line end included, through the same row parser on the host (pb200_input_csv_row_host;
+    tests): (dim_id, ds_ns, quantity or None), or None when the parser refuses the line."""
+    import ctypes
+    dim, ds, q, qv = ctypes.c_int32(), ctypes.c_int64(), ctypes.c_int32(), ctypes.c_int32()
+    rc = L.load().pb200_input_csv_row_host(line, len(line), ctypes.addressof(dim), ctypes.addressof(ds),
+                                           ctypes.addressof(q), ctypes.addressof(qv))
+    if rc < 0:
+        raise ValueError("pb200_input_csv_row_host: bad argument")
+    return (dim.value, ds.value, q.value if qv.value else None) if rc == 1 else None
+
+
 def predict_batch_host(ctx: L.Context, opts: L.Options, fitted: FittedBatch, future_ds: np.ndarray,
                        floor: np.ndarray, cap: np.ndarray, seed: int = 0, intervals: bool = True) -> ForecastBatch:
     """pb200_predict_host.  ``floor`` / ``cap`` per model as the scorer reads them back from

@@ -7,6 +7,7 @@
 #include "mc_kernel.cuh"
 #include "newton_kernel.cuh"
 #include "csv_kernel.cuh"
+#include "csv_reader.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -988,6 +989,101 @@ PB200_API int32_t pb200_forecast_csv_row_host(int32_t series_id, int32_t dim_id,
     char* e = pb200::csv::put_row(out, series_id, dim_id, ds_ns, quantity, created, created_len);
     const int n = (int)(e - out);
     return n == pb200::csv::row_len(series_id, dim_id, quantity, created_len) ? n : -1;
+}
+
+// ---- modeler input CSV parsed on the device (csv_reader.cuh) ----
+static_assert(PB200_INPUT_CSV_TILE == pb200::csvin::TILE, "tile size of the count / index passes");
+
+static int input_args(pb200::csvin::InArgs& a, const uint8_t* text, int64_t n_bytes) {
+    memset(&a, 0, sizeof a);
+    if (n_bytes < 0) return fail(PB200_E_ARG, "sizes");
+    if (n_bytes && !text) return fail(PB200_E_ARG, "null pointer");
+    if ((uintptr_t)text % 16) return fail(PB200_E_ARG, "d_text must be 16-byte aligned");
+    a.text = text;
+    a.n_bytes = n_bytes;
+    return PB200_OK;
+}
+
+static int input_tile_grid(const pb200_ctx* c, int64_t n_bytes) {
+    const int64_t tiles = (n_bytes + pb200::csvin::TILE - 1) / pb200::csvin::TILE;
+    return (int)std::min<int64_t>((tiles + 7) / 8, (int64_t)c->sms * 8);
+}
+
+PB200_API int pb200_input_csv_count_device(pb200_ctx* c, const uint8_t* d_text, int64_t n_bytes, int64_t* d_tile_count) {
+    if (!c) return fail(PB200_E_ARG, "ctx is null");
+    pb200::csvin::InArgs a;
+    int rc = input_args(a, d_text, n_bytes);
+    if (rc) return rc;
+    if (n_bytes == 0) return PB200_OK;
+    if (!d_tile_count) return fail(PB200_E_ARG, "null pointer");
+    CK(cudaSetDevice(c->device));
+    a.tile_count = (long long*)d_tile_count;
+    pb200::csvin::input_count_kernel<<<input_tile_grid(c, n_bytes), 256, 0, c->stream>>>(a);
+    CK(cudaGetLastError());
+    c->launches++;
+    return PB200_OK;
+}
+
+PB200_API int pb200_input_csv_index_device(pb200_ctx* c, const uint8_t* d_text, int64_t n_bytes, const int64_t* d_tile_off,
+                                           int64_t* d_row_end) {
+    if (!c) return fail(PB200_E_ARG, "ctx is null");
+    pb200::csvin::InArgs a;
+    int rc = input_args(a, d_text, n_bytes);
+    if (rc) return rc;
+    if (n_bytes == 0) return PB200_OK;
+    if (!d_tile_off || !d_row_end) return fail(PB200_E_ARG, "null pointer");
+    CK(cudaSetDevice(c->device));
+    a.tile_off = (const long long*)d_tile_off;
+    a.row_end = (long long*)d_row_end;
+    pb200::csvin::input_index_kernel<<<input_tile_grid(c, n_bytes), 256, 0, c->stream>>>(a);
+    CK(cudaGetLastError());
+    c->launches++;
+    return PB200_OK;
+}
+
+PB200_API int pb200_input_csv_parse_device(pb200_ctx* c, const uint8_t* d_text, const int64_t* d_row_end, int64_t n_rows,
+                                           const int64_t* d_file_start, const int32_t* d_file_sid, int32_t n_files,
+                                           int32_t* d_series_id, int32_t* d_dim_id, int64_t* d_ds_ns, int32_t* d_quantity,
+                                           uint8_t* d_quantity_valid, int64_t* d_refused) {
+    if (!c) return fail(PB200_E_ARG, "ctx is null");
+    if (n_rows < 0 || n_files < 0 || (n_rows > 0 && n_files == 0)) return fail(PB200_E_ARG, "sizes");
+    if (!d_refused) return fail(PB200_E_ARG, "null pointer");
+    CK(cudaSetDevice(c->device));
+    CK(cudaMemsetAsync(d_refused, 0, 8, c->stream));
+    CK(cudaMemsetAsync(d_refused + 1, 0xFF, 8, c->stream));
+    if (n_rows == 0) return PB200_OK;
+    if (!d_row_end || !d_file_start || !d_file_sid || !d_series_id || !d_dim_id || !d_ds_ns || !d_quantity || !d_quantity_valid)
+        return fail(PB200_E_ARG, "null pointer");
+    pb200::csvin::InArgs a;
+    int rc = input_args(a, d_text, 1);
+    if (rc) return rc;
+    a.row_end = (long long*)d_row_end;
+    a.n_rows = n_rows;
+    a.file_start = (const long long*)d_file_start;
+    a.file_sid = d_file_sid;
+    a.n_files = n_files;
+    a.sid = d_series_id;
+    a.dim = d_dim_id;
+    a.ds = (long long*)d_ds_ns;
+    a.qty = d_quantity;
+    a.qty_valid = d_quantity_valid;
+    a.refused = (unsigned long long*)d_refused;
+    const int64_t warps = (n_rows + 31) / 32;
+    const int grid = (int)std::min<int64_t>((warps + 3) / 4, (int64_t)c->sms * 16);
+    pb200::csvin::input_parse_kernel<<<grid, 128, 0, c->stream>>>(a);
+    CK(cudaGetLastError());
+    c->launches++;
+    return PB200_OK;
+}
+
+PB200_API int32_t pb200_input_csv_row_host(const char* line, int64_t len, int32_t* dim_id, int64_t* ds_ns, int32_t* quantity,
+                                           int32_t* quantity_valid) {
+    if (len < 0 || (len && !line) || !dim_id || !ds_ns || !quantity || !quantity_valid) return -1;
+    const unsigned char* p = (const unsigned char*)line;
+    bool qv = false;
+    const bool ok = pb200::csvin::parse_row(p, p + len, *dim_id, *ds_ns, *quantity, qv);
+    *quantity_valid = ok && qv;
+    return ok ? 1 : 0;
 }
 
 }  // extern "C"

@@ -54,6 +54,16 @@ __host__ __device__ __forceinline__ void civil_from_days(int64_t z, int& y, int&
     y = (int)(yoe + era * 400) + (m <= 2 ? 1 : 0);
 }
 
+// day count since 1970-01-01 of a civil date (proleptic Gregorian; the inverse of civil_from_days, any year >= 1 here)
+__host__ __device__ __forceinline__ int64_t days_from_civil(int y, int m, int d) {
+    y -= m <= 2;
+    const int era = y / 400;                         // y >= 0: no floor correction needed
+    const unsigned yoe = (unsigned)(y - era * 400);
+    const unsigned doy = (153u * (unsigned)(m > 2 ? m - 3 : m + 9) + 2u) / 5u + (unsigned)d - 1u;
+    const unsigned doe = yoe * 365u + yoe / 4u - yoe / 100u + doy;
+    return (int64_t)era * 146097 + (int64_t)doe - 719468;
+}
+
 __host__ __device__ __forceinline__ int row_len(int32_t sid, int32_t did, int32_t qty, int created_len) {
     return created_len + int_len(sid) + int_len(did) + int_len(qty) + FIXED_BYTES;
 }

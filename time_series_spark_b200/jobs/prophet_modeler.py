@@ -30,8 +30,9 @@ import pyarrow.parquet as pq
 from .. import _lib as L
 from .. import batched, model_record
 from .. import dist as pdist
-from ..frame import Frame
-from ..pack import pack_groups, pack_groups_cuda
+from .. import csv_input
+from ..frame import DeviceColumns, Frame
+from ..pack import pack_device_columns, pack_groups_cuda
 
 # reference prophet_modeler.py:12-17 (Spark StructType -> Arrow)
 MODEL_INPUT_SCHEMA = pa.schema([
@@ -49,6 +50,10 @@ MODEL_OUTPUT_SCHEMA = pa.schema([
     pa.field("cap", pa.float32(), True),
     pa.field("model", pa.binary(), True),
 ])
+
+# Whether io.reader = auto takes the GPU reader.  It does so only once a measurement on the B200
+# (tools/bench_reader.py) shows it faster than Arrow on the 16 000-series config-#3 tree; that run has not been made yet.
+AUTO_READS_ON_GPU = False
 
 _contexts = {}
 
@@ -85,15 +90,31 @@ class _ModelTimeSeriesOp:
 
     def apply_batched(self, table: pa.Table, keys) -> pa.Table:
         execution_time = time.time()
+        ctx = self._start(keys)
+        # upload, then group + sort on the GPU (two radix sorts), ds / y stay in HBM for the fit
+        return self._fit_packed(pack_groups_cuda(table, device=f"cuda:{ctx.device}"), execution_time)
+
+    def apply_device_columns(self, cols: DeviceColumns, keys) -> pa.Table:
+        """The same for a frame the GPU input reader left in HBM: no copy back to the host and up again."""
+        execution_time = time.time()
+        self._start(keys)
+        return self._fit_packed(pack_device_columns(cols.series_id, cols.dim_id, cols.ds, cols.y, cols.y_valid == 0),
+                                execution_time)
+
+    @staticmethod
+    def _start(keys) -> L.Context:
         if list(keys) != ["series_id", "dim_id"]:
             raise ValueError("model_time_series groups by ('series_id', 'dim_id')")
+        ctx = get_context()
+        import torch
+        torch.cuda.set_device(ctx.device)
+        return ctx
+
+    def _fit_packed(self, pk, execution_time: float) -> pa.Table:
+        import torch
         floor = self.config["model"]["floor"]
         cap_multiplier = self.config["model"]["cap_multiplier"]
         ctx = get_context()
-        # group + sort on the GPU (two radix sorts), ds / y stay in HBM for the fit
-        import torch
-        torch.cuda.set_device(ctx.device)
-        pk = pack_groups_cuda(table, device=f"cuda:{ctx.device}")
         torch.cuda.synchronize()
         t_pack = time.time()
         rank, ws, _ = pdist.world()
@@ -177,6 +198,17 @@ def rank_local_files(dset, rank: int, world_size: int):
     return [p for s in sids[lo:hi] for p in sorted(by_sid[s][1])]
 
 
+def input_csv_format() -> pads.CsvFileFormat:
+    """How the Arrow reader parses one input file: header-less ``dim_id,start_time,quantity`` at the types of
+    MODEL_INPUT_SCHEMA."""
+    names = [f.name for f in MODEL_INPUT_SCHEMA if f.name != "series_id"]
+    return pads.CsvFileFormat(
+        read_options=pacsv.ReadOptions(column_names=names),
+        convert_options=pacsv.ConvertOptions(
+            column_types={f.name: f.type for f in MODEL_INPUT_SCHEMA if f.name != "series_id"},
+            timestamp_parsers=["%Y-%m-%d %H:%M:%S", pacsv.ISO8601]))
+
+
 def model_time_series(config):
     """Model time series per dimensions (series_id, dim_id)  -- reference prophet_modeler.py:22-87."""
     return _ModelTimeSeriesOp(config)
@@ -192,16 +224,18 @@ class ProphetModeler:
     def read_input_dataframe(self, spark=None) -> Frame:
         """Header-less CSV ``dim_id,timestamp,quantity`` under hive dirs ``series_id=<int>/``
         (reference :102-116; fixture tests/fixtures/model-input).  Returns columns
-        series_id, dim_id, ds, y."""
-        pdist.size_host_pools()             # pyarrow threads = this rank's share of the lease, not os.cpu_count()
+        series_id, dim_id, ds, y.
+
+        ``io.reader`` picks the parser: ``arrow`` (pyarrow on the host), ``gpu`` (csrc/csv_reader.cuh; raises
+        ValueError for an input it does not take) or ``auto`` (the default: the GPU reader when AUTO_READS_ON_GPU and
+        CUDA is usable, else -- and for any input the GPU reader does not take -- Arrow).  Both give the same table."""
+        reader = (self.config["io"].get("reader") or "auto")
+        if reader not in ("auto", "gpu", "arrow"):
+            raise ValueError("io.reader must be 'auto', 'gpu' or 'arrow'")
+        threads = pdist.size_host_pools()   # pyarrow threads = this rank's share of the lease, not os.cpu_count()
         path = self.config["io"]["input"]
         part = pads.partitioning(pa.schema([("series_id", pa.int32())]), flavor="hive")
-        names = [f.name for f in MODEL_INPUT_SCHEMA if f.name != "series_id"]
-        fmt = pads.CsvFileFormat(
-            read_options=pacsv.ReadOptions(column_names=names),
-            convert_options=pacsv.ConvertOptions(
-                column_types={f.name: f.type for f in MODEL_INPUT_SCHEMA if f.name != "series_id"},
-                timestamp_parsers=["%Y-%m-%d %H:%M:%S", pacsv.ISO8601]))
+        fmt = input_csv_format()
         dset = pads.dataset(path, format=fmt, partitioning=part, exclude_invalid_files=False,
                             ignore_prefixes=[".", "_"])
         # Rank-local ingestion (SURVEY 8e): a group never spans two ``series_id=`` directories, so under torchrun each
@@ -220,6 +254,13 @@ class ProphetModeler:
                     return Frame(empty)
                 dset = pads.dataset(mine, format=fmt, partitioning=part, partition_base_dir=path,
                                     exclude_invalid_files=False)
+        if reader == "gpu" or (reader == "auto" and AUTO_READS_ON_GPU):
+            cols, why = csv_input.read_device(dset, get_context, threads)
+            if cols is not None:
+                return Frame(device_columns=cols)
+            if reader == "gpu":
+                raise ValueError("io.reader = 'gpu' cannot read this input: " + why)
+            print(f"Reading the input with Arrow: {why}")
         tbl = dset.to_table(columns=["series_id", "dim_id", "start_time", "quantity"])
         tbl = tbl.rename_columns(["series_id", "dim_id", "ds", "y"])
         return Frame(tbl)

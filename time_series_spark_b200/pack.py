@@ -8,6 +8,7 @@ still count for ``history_dates.max()`` (the anchor of make_future_dataframe).
 """
 from __future__ import annotations
 
+import bisect
 from dataclasses import dataclass
 
 import numpy as np
@@ -134,39 +135,40 @@ _SLOT_BYTES = 32 << 20
 _slots = {}            # device index -> (two pinned byte tensors, two CUDA events): the H2D staging ring
 
 
-def _device_column(col, arrow_type, dev):
-    """A null-free primitive Arrow column (ChunkedArray) -> one contiguous device tensor.  The chunks are memcpy'd
-    back to back into a small ring of pinned slots and DMA'd from there while the next slot fills: the only host pass
-    over the column is that memcpy (no combine_chunks, no pageable cudaMemcpy of a 64-bit key built in numpy -- the
-    two things that made the pack 42 % of the modeler job's wall time in profiles/r2u_e2e_stage_breakdown.log)."""
+def ring_upload(out, fill) -> None:
+    """Fills the contiguous device tensor ``out`` through a small ring of pinned slots: ``fill(dst, lo, hi)`` writes
+    bytes [lo, hi) of ``out``'s contents into the pinned uint8 numpy array ``dst``, and each slot is DMA'd to the
+    device while the next one fills.  The copies are queued on the current stream."""
     import torch
-    tdtype = {pa.int64(): torch.int64, pa.int32(): torch.int32, pa.float64(): torch.float64}[arrow_type]
-    width = 8 if arrow_type != pa.int32() else 4
-    n = len(col)
-    out = torch.empty(n, dtype=tdtype, device=dev)
+    dev = out.device
     ring = _slots.get(dev.index)
     if ring is None:
         ring = ([torch.empty(_SLOT_BYTES, dtype=torch.uint8, pin_memory=True) for _ in range(2)],
                 [torch.cuda.Event() for _ in range(2)])
         _slots[dev.index] = ring
     bufs, evs = ring
-    cap = _SLOT_BYTES // width
-    views = [b.view(tdtype) for b in bufs]
-    np_views = [v.numpy() for v in views]
-    cur, fill, done = 0, 0, 0
-    evs[0].synchronize()
-    evs[1].synchronize()
+    dst = out.view(torch.uint8)
+    n = dst.numel()
+    slot = bufs[0].numel()
+    cur = 0
+    for lo in range(0, n, slot):
+        hi = min(n, lo + slot)
+        evs[cur].synchronize()              # the slot about to be refilled has left for the device
+        fill(bufs[cur].numpy()[:hi - lo], lo, hi)
+        dst[lo:hi].copy_(bufs[cur][:hi - lo], non_blocking=True)
+        evs[cur].record()
+        cur ^= 1
 
-    def flush():
-        nonlocal cur, fill, done
-        if fill:
-            out[done:done + fill].copy_(views[cur][:fill], non_blocking=True)
-            evs[cur].record()
-            done += fill
-            cur ^= 1
-            fill = 0
-            evs[cur].synchronize()          # the slot about to be refilled has left for the device
 
+def _device_column(col, arrow_type, dev):
+    """A null-free primitive Arrow column (ChunkedArray) -> one contiguous device tensor.  The chunks are memcpy'd
+    back to back into the pinned ring (ring_upload): the only host pass over the column is that memcpy (no
+    combine_chunks, no pageable cudaMemcpy of a 64-bit key built in numpy -- the two things that made the pack 42 % of
+    the modeler job's wall time in profiles/r2u_e2e_stage_breakdown.log)."""
+    import torch
+    tdtype = {pa.int64(): torch.int64, pa.int32(): torch.int32, pa.float64(): torch.float64}[arrow_type]
+    out = torch.empty(len(col), dtype=tdtype, device=dev)
+    pieces, starts = [], [0]
     for ch in col.chunks if isinstance(col, pa.ChunkedArray) else [col]:
         if len(ch) == 0:
             continue
@@ -174,24 +176,25 @@ def _device_column(col, arrow_type, dev):
             ch = ch.view(pa.int64())
         elif ch.type != arrow_type:
             ch = pc.cast(ch, arrow_type, safe=False)
-        src = ch.to_numpy(zero_copy_only=True)
-        a = 0
-        while a < src.size:
-            m = min(src.size - a, cap - fill)
-            np_views[cur][fill:fill + m] = src[a:a + m]
-            fill += m
-            a += m
-            if fill == cap:
-                flush()
-    flush()
+        pieces.append(ch.to_numpy(zero_copy_only=True).view(np.uint8))
+        starts.append(starts[-1] + pieces[-1].size)
+
+    def fill(dst, lo, hi):
+        k, o = bisect.bisect_right(starts, lo) - 1, 0
+        while o < dst.size:
+            a = lo + o - starts[k]
+            m = min(dst.size - o, pieces[k].size - a)
+            dst[o:o + m] = pieces[k][a:a + m]
+            o += m
+            k += 1
+
+    ring_upload(out, fill)
     return out
 
 
 def pack_groups_cuda(table: pa.Table, device=None, keys=("series_id", "dim_id"), ds_col="ds", y_col="y"):
     """GPU version of :func:`pack_groups` (SURVEY 8f-2): the columns go to HBM as they are (32-bit ids and y, 64-bit
-    ds), the sort key is formed there and the (series_id, dim_id, ds) sort of the whole frame runs on the B200 as two
-    stable radix sorts (``torch.sort`` -- plumbing, not a hand-written kernel; skipped when the frame already is in
-    that order, as a hive-partitioned input written per series is).  ``ds`` / ``y`` stay resident in HBM for
+    ds) and :func:`pack_device_columns` groups and sorts them there.  ``ds`` / ``y`` stay resident in HBM for
     ``pb200_fit_device``.  Returns a PackedGroups whose ``ds`` / ``y`` are CUDA tensors; ids, offsets and last_ds are
     host numpy arrays.  Null ``y`` rows are dropped exactly as on the host path."""
     import torch
@@ -222,11 +225,28 @@ def pack_groups_cuda(table: pa.Table, device=None, keys=("series_id", "dim_id"),
     k0 = _device_column(table[keys[0]], pa.int32(), dev)
     k1 = _device_column(table[keys[1]], pa.int32(), dev)
     y_t = _device_column(ycol, pa.int32() if integral else pa.float64(), dev)
-    if not integral:
+    return pack_device_columns(k0, k1, ds_t, y_t, y_null)
+
+
+def pack_device_columns(k0, k1, ds_t, y_t, y_null=None) -> PackedGroups:
+    """The device half of :func:`pack_groups_cuda`: int32 series_id / dim_id, int64 ns ds and int32 or float64 y, CUDA
+    tensors of one length on one device, in input row order; ``y_null`` marks null y rows (None, a host bool array or
+    a CUDA bool tensor).  The sort key is formed on the device and the (series_id, dim_id, ds) sort of the whole frame
+    runs on the B200 as two stable radix sorts (``torch.sort`` -- plumbing, not a hand-written kernel; skipped when the
+    frame already is in that order, as a hive-partitioned input written per series is).  Float y NaNs count as
+    nulls.  The input tensors may be consumed."""
+    import torch
+    dev = ds_t.device
+    if ds_t.numel() == 0:
+        z = np.zeros(0, np.int32)
+        y_dtype = np.int32 if y_t.dtype == torch.int32 else np.float64
+        return PackedGroups(z, z, np.zeros(1, np.int64), np.zeros(0, np.int64), np.zeros(0, y_dtype), np.zeros(0, np.int64),
+                            np.zeros(0, np.int64))
+    if y_null is not None and not isinstance(y_null, torch.Tensor):
+        y_null = torch.from_numpy(np.asarray(y_null, dtype=bool)).to(dev)
+    if y_t.is_floating_point():
         nan = torch.isnan(y_t)
-        if bool(nan.any()):
-            nan_h = nan.cpu().numpy()
-            y_null = nan_h if y_null is None else (y_null | nan_h)
+        y_null = nan if y_null is None else (y_null | nan)
     # one signed 64-bit sort key: series_id in the high word, dim_id biased by 2^31 in the low word, so that the
     # signed order of the key is the (series_id, dim_id) order of the host path's lexsort for negative ids too
     key = (k0.to(torch.int64) << 32) | (k1.to(torch.int64) + (1 << 31))
@@ -246,8 +266,8 @@ def pack_groups_cuda(table: pa.Table, device=None, keys=("series_id", "dim_id"),
     n_rows_in = (ends - starts).cpu().numpy().astype(np.int64)
     gkeys = key[starts].cpu().numpy()
     sid, did = (gkeys >> 32).astype(np.int32), ((gkeys & 0xFFFFFFFF) - (1 << 31)).astype(np.int32)
-    if y_null is not None and y_null.any():
-        keep = ~torch.from_numpy(y_null).to(dev)
+    if y_null is not None and bool(y_null.any()):
+        keep = ~y_null
         if order is not None:
             keep = keep[order]
         grp_id = torch.cumsum(new_grp.to(torch.int64), 0) - 1

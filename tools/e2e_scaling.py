@@ -1,9 +1,9 @@
 """Modeler job end to end on a config-#3-shaped hive-partitioned CSV, timed per stage, for 1..N ranks (SURVEY 8e:
 "rank r reads only its row range").  Usage:
     python tools/e2e_scaling.py make <dir> <n_series> [T]                 # write the input once
-    python -m torch.distributed.run --nproc-per-node N ... tools/e2e_scaling.py run <dir>
-`run` prints one JSON line on rank 0: wall time of read / fit (pack + GPU fit + encode) / write, max over ranks,
-and what each rank read."""
+    python -m torch.distributed.run --nproc-per-node N ... tools/e2e_scaling.py run <dir> [auto|gpu|arrow]
+`run` reads the input with the given io.reader (default: the config's) and prints one JSON line on rank 0: wall time
+of read / fit (pack + GPU fit + encode) / write, max over ranks, and what each rank read."""
 import json
 import os
 import sys
@@ -38,12 +38,14 @@ def make(d, n, T=1440):
     print(f"wrote {n} series x {T} points under {inp} in {time.time() - t0:.1f} s")
 
 
-def run(d):
+def run(d, reader=None):
     import torch
     import yaml
     from time_series_spark_b200 import dist as pdist
     from time_series_spark_b200.jobs.prophet_modeler import ProphetModeler, model_time_series
     cfg = yaml.safe_load(open(os.path.join(d, "modeler.yaml")))
+    if reader:
+        cfg["io"]["reader"] = reader
     pdist.init_process_group()
     rank, ws, local = pdist.world()
     torch.cuda.set_device(local)
@@ -77,7 +79,7 @@ def run(d):
         allc = [cnt]
     if rank == 0:
         r, f, w, t, opk, ofi, oen = [float(x) for x in vals.tolist()]
-        print(json.dumps({"ranks": ws, "rank_local_input": bool(getattr(job, "rank_local_input", False)),
+        print(json.dumps({"ranks": ws, "reader": cfg["io"].get("reader", "auto"), "rank_local_input": bool(getattr(job, "rank_local_input", False)),
                           "read_s": r, "fit_s": f, "write_s": w, "total_s": t,
                           "fit_stage": {"pack_upload_group_sort_s": opk, "gpu_fit_and_d2h_s": ofi, "encode_records_s": oen},
                           "rows_read_by_rank": [int(c[0]) for c in allc], "models_by_rank": [int(c[1]) for c in allc]}))
@@ -90,4 +92,4 @@ if __name__ == "__main__":
     if sys.argv[1] == "make":
         make(sys.argv[2], int(sys.argv[3]), int(sys.argv[4]) if len(sys.argv) > 4 else 1440)
     else:
-        run(sys.argv[2])
+        run(sys.argv[2], sys.argv[3] if len(sys.argv) > 3 else None)
